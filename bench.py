@@ -6,6 +6,8 @@ synthetic tokens, random-init weights.  Parallel layout per N: 1 -> single GPU; 
 8 -> dp2 x mp2 x pp2.  Weak scaling: 4 sequences of 4096 tokens per GPU per step.
 
   python bench.py --gpus 1 --steps 5 --warmup 3
+  python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR   -> also writes the last step's loss and sampled parameters as .npy
+                                                                       files; inputs are seeded, so two builds compare file by file
   python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29511 bench.py --gpus 8 ...
   python bench.py --impl reference ...   -> {"impl": "reference", "unavailable": ...}
   python bench.py --impl library ...     -> same model and engine with the spec's hot ops on LIBRARY kernels (cuBLAS GEMMs, cuDNN / flash
@@ -49,6 +51,8 @@ def parse():
     ap.add_argument("--no-comm-calibration", action="store_true")
     ap.add_argument("--recompute-skip", type=int, default=-1,
                     help="N=1 only: number of trailing decoder layers that keep their activations (default: as many as fit in HBM)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the last step's loss and a fixed sample of the updated parameters as DIR/<name>.npy")
     args = ap.parse_args()
     # auto-tuner trials (paddle_b200.distributed.launch --auto_tuner_json / distributed.auto_tuner.AutoTuner.tune): the candidate arrives in the
     # environment and overrides the layout flags; sharding candidates are not a bench.py layout and leave the flags untouched
@@ -120,6 +124,29 @@ def layout_for(n):
     # (dp, mp, pp): sub-meshes of the 8-GPU dp2 x mp2 x pp2 layout BASELINE.json names; at 4 GPUs dp2 x mp2 measured 14 % faster
     # than mp2 x pp2 (no pipeline bubble, larger micro-batches)
     return {1: (1, 1, 1), 2: (1, 2, 1), 4: (2, 2, 1), 8: (2, 2, 2)}.get(n, (n, 1, 1))
+
+
+DUMP_BUDGET_BYTES = 48 << 20   # all parameter samples together; stays under 64 MB whatever the model size
+
+
+def dump_outputs(out_dir, loss, model):
+    """Write what a caller of the training step holds after the last timed step, so that two builds can be compared output for
+    output: `loss.npy` (float64) and, per parameter, `<parameter name>.npy` (float32) with the whole parameter when it is small,
+    otherwise the values at positions drawn by a generator seeded with the parameter's index (the same positions in every run)."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    loss = loss.detach().float().item() if isinstance(loss, torch.Tensor) else float(loss)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([loss], dtype=np.float64))
+    params = list(model.named_parameters())
+    per_param = max(1, DUMP_BUDGET_BYTES // 4 // max(1, len(params)))
+    for i, (name, p) in enumerate(params):
+        flat = p.detach().as_subclass(torch.Tensor).reshape(-1)
+        if flat.numel() > per_param:
+            idx = torch.randint(0, flat.numel(), (per_param,), generator=torch.Generator().manual_seed(i)).sort().values
+            flat = flat[idx.to(flat.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), flat.float().cpu().numpy())
 
 
 def exposed_comm_report(regions, args, cfg, mp, pp, dp, accumulate, n, local_rank, ms_per_step):
@@ -434,6 +461,8 @@ def main():
     out["model_tflops_per_gpu"] = round(value * flops_per_token / n / 1e12, 1)
     if peaks.get("bf16_tflops_sustained"):
         out["mfu_of_measured_sustained_peak"] = round(out["model_tflops_per_gpu"] / peaks["bf16_tflops_sustained"], 3)
+    if args.dump_outputs and rank == 0:   # with several ranks: rank 0's loss and its share of the parameters
+        dump_outputs(args.dump_outputs, last, model)
     if rank == 0:
         print(json.dumps(out))
     if n > 1:

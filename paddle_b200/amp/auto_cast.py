@@ -11,6 +11,7 @@ import contextlib
 import torch
 
 from ..framework import dtype as _dt
+from ..framework.place import _default_device
 
 WHITE_LIST = {"conv2d", "einsum", "matmul", "matmul_v2", "max_pool2d_with_index", "mul", "fused_gemm_epilogue", "linear", "flash_attn"}
 BLACK_LIST = {"exp", "square", "log", "mean", "sum", "cos_sim", "softmax", "softmax_with_cross_entropy", "sigmoid_cross_entropy_with_logits",
@@ -23,8 +24,7 @@ def fp32_guard(op, *tensors):
     """For white-list ops that the user moved to `custom_black_list`: returns (context, tensors cast to fp32) so the op runs
     outside autocast; a no-op context and the tensors unchanged otherwise."""
     if _state["enabled"] and op in _state["black"]:
-        dev = "cuda" if torch.cuda.is_available() else "cpu"
-        return torch.autocast(device_type=dev, enabled=False), tuple(t.float() if isinstance(t, torch.Tensor) and t.is_floating_point() else t for t in tensors)
+        return torch.autocast(device_type=_default_device().type, enabled=False), tuple(t.float() if isinstance(t, torch.Tensor) and t.is_floating_point() else t for t in tensors)
     if _state["enabled"] and _state["level"] == "O2" and len(tensors) >= 2:
         # O2: parameters are low precision; an fp32 activation (typically the model input) meeting them is cast down, like the
         # reference's O2 autocast of white-list op inputs.  Only reached on paths where the dtypes would otherwise clash.
@@ -77,7 +77,7 @@ def auto_cast(enable=True, custom_white_list=None, custom_black_list=None, level
     active = enable and level != "O0"
     _state.update(enabled=active, level=level if active else "O0", dtype=d if active else torch.float32,
                   black=frozenset(custom_black_list or ()) if active else frozenset(), white=frozenset(custom_white_list or ()) if active else frozenset())
-    dev = "cuda" if torch.cuda.is_available() else "cpu"
+    dev = _default_device().type   # the current device (paddle.set_device), like the reference's expected place
     try:
         if active and level in ("O1", "OD"):
             if dev == "cpu" and d == torch.float16:

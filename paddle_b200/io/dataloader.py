@@ -13,6 +13,7 @@ import threading
 import numpy as np
 import torch
 
+from ..framework.place import _default_device
 from ..tensor import Tensor
 from .dataset import IterableDataset
 from .sampler import BatchSampler
@@ -109,12 +110,13 @@ class DataLoader:
         else:
             self.batch_sampler = BatchSampler(dataset, shuffle=shuffle, batch_size=batch_size, drop_last=drop_last)
         self._device = None
+        on_gpu = _default_device().type == "cuda"     # the current device (paddle.set_device), not merely a visible GPU
         if device_prefetch is None:
-            device_prefetch = torch.cuda.is_available() and use_buffer_reader
+            device_prefetch = on_gpu and use_buffer_reader
         if device_prefetch and torch.cuda.is_available():
             self._device = torch.device("cuda", torch.cuda.current_device())
         self._ring = None
-        self._pin = pin_memory if pin_memory is not None else torch.cuda.is_available()
+        self._pin = pin_memory if pin_memory is not None else on_gpu
 
     def __len__(self):
         if self._iterable:

@@ -53,13 +53,14 @@ def _lower(layer, config):
     import torch
 
     from . import jit
+    from .framework.place import _default_device
     from .tensor import Tensor
 
     if config.precision_mode in (PrecisionMode.FP16, PrecisionMode.BF16) and hasattr(layer, "to"):
         layer.to(dtype=config.precision_mode)
     layer.eval() if hasattr(layer, "eval") else None
     profiles = [inp.generate_input_data() for inp in config.inputs]
-    on_gpu = torch.cuda.is_available()
+    on_gpu = _default_device().type == "cuda"     # the current device (paddle.set_device), not merely a visible GPU
     fn = jit.to_static(layer) if (config.use_cuda_graph and on_gpu) else layer
     with torch.no_grad():
         for which in (0, 2, 1, 1, 1):   # min, max, then the optimum often enough for the capture to happen
