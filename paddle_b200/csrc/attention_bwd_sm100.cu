@@ -16,11 +16,11 @@
 // TMEM columns: [0,128) S then dQ^T, [128,256) dP, [256,384) dV, [384,512) dK.
 #include <cuda.h>
 #include <cstdio>
-#include <string>
 
 #include "include/b200_common.cuh"
 #include "include/b200_ops.h"
 #include "include/b200_ptx.cuh"
+#include "include/b200_tcgen05_host.h"
 
 namespace b200 {
 namespace attn_bwd {
@@ -40,16 +40,6 @@ constexpr uint32_t S_COL = 0, DP_COL = 128, DV_COL = 256, DK_COL = 384;
 //   MN-major use  (rows = K index, inner = M or N):   K step k (16 rows)                 -> +k*2048,         LBO HALF (next 64 M/N), SBO 1024
 __device__ __forceinline__ uint64_t desc_kmajor(uint32_t tile, int kb, int k) { return make_smem_desc(tile + kb * HALF_BYTES + k * 32, 16, 1024); }
 __device__ __forceinline__ uint64_t desc_mnmajor(uint32_t tile, int kk) { return make_smem_desc(tile + kk * 2048, HALF_BYTES, 1024); }
-
-template <typename T> __device__ __forceinline__ uint32_t pack2(float a, float b);
-template <> __device__ __forceinline__ uint32_t pack2<__nv_bfloat16>(float a, float b) {
-  const __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<const uint32_t*>(&v);
-}
-template <> __device__ __forceinline__ uint32_t pack2<__half>(float a, float b) {
-  const __half2 v = __floats2half2_rn(a, b);
-  return *reinterpret_cast<const uint32_t*>(&v);
-}
 
 struct Params {
   int b, sq, sk, h, hk;
@@ -98,17 +88,16 @@ bwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CU
   const int total = tiles_per_head * group;    // iteration it -> (query head = kv_head*group + it / tiles_per_head, m tile = m_first + it % tiles_per_head)
 
   if (warp == 8 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_q) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_k) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_v) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_do) : "memory");
+    tma_prefetch_desc(&map_q);
+    tma_prefetch_desc(&map_k);
+    tma_prefetch_desc(&map_v);
+    tma_prefetch_desc(&map_do);
     mbar_init(kv_full, 1); mbar_init(qdo_full, 1); mbar_init(qdo_empty, 1); mbar_init(s_full, 1); mbar_init(s_free, 8);
     mbar_init(pds_full, 8); mbar_init(dq_full, 1); mbar_init(acc_done, 1);
     fence_barrier_init();
     fence_proxy_async();
   } else if (warp == 9) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_ptr)), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(smem_u32((const void*)tmem_ptr), TMEM_COLS);
   }
   tc_fence_before();
   __syncthreads();
@@ -218,8 +207,8 @@ bwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CU
           }
           const int col = c * 32 + q8 * 8;              // key index inside this 64-key half
           const uint32_t off = half * HALF_BYTES + rl * 128 + (((col >> 3) ^ (rl & 7)) << 4);
-          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(sP + off), "r"(up[0]), "r"(up[1]), "r"(up[2]), "r"(up[3]) : "memory");
-          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(sDS + off), "r"(ud[0]), "r"(ud[1]), "r"(ud[2]), "r"(ud[3]) : "memory");
+          st_shared_v4(sP + off, up[0], up[1], up[2], up[3]);
+          st_shared_v4(sDS + off, ud[0], ud[1], ud[2], ud[3]);
         }
       }
       fence_proxy_async();
@@ -266,16 +255,16 @@ bwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CU
       asm volatile("bar.sync 1, 256;" ::: "memory");      // both softmax warpgroups: the whole [128][128] fp32 tile is in smem (and it is our turn)
       if (half == 0 && m0 + rl < p.sq) {
         float* dst = p.dq + (int64_t)batch * p.dq_sb + (int64_t)(m0 + rl) * p.dq_ss + (int64_t)head * p.dq_sh;
-        asm volatile("cp.reduce.async.bulk.global.shared::cta.bulk_group.add.f32 [%0], [%1], 512;" ::"l"(dst), "r"(sDQ + (uint32_t)rl * 512u) : "memory");
+        bulk_reduce_add_f32<512>(dst, sDQ + (uint32_t)rl * 512u);
       }
-      asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+      bulk_commit();
       if (sem) {
-        asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");      // the adds have been performed, not just read from smem
+        bulk_wait<0>();                                    // the adds have been performed, not just read from smem
         __threadfence();
         asm volatile("bar.sync 1, 256;" ::: "memory");
         if (threadIdx.x == 0) asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(sem), "r"(n_tile + 1) : "memory");
       } else {
-        asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // the tile in shared memory may be overwritten
+        bulk_wait_read<0>();                               // the tile in shared memory may be overwritten
       }
       __syncwarp();
       if (lane == 0) mbar_arrive(s_free);            // 8 warp arrivals
@@ -322,7 +311,7 @@ bwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CU
   __syncthreads();
   if (warp == 9) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    tmem_dealloc(tmem_base, TMEM_COLS);
   }
 }
 
@@ -350,47 +339,13 @@ __global__ void delta_kernel(const T* __restrict__ o, const T* __restrict__ d_o,
   if (lane == 0) delta[(bb * h + head) * sq + sidx] = acc;
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)p;
-  }
-  return fn;
-}
+// 4-D map {d, s, h, b} over a strided [B,S,H,D] view (strides in elements), box {64, 128, 1, 1}, 128B swizzle
 static bool make_map4(CUtensorMap* out, const void* ptr, int d, int s, int h, int b, int64_t ss, int64_t sh, int64_t sb, int dtype) {
-  bind_primary_context();
-  EncodeTiledFn enc = get_encode();
-  if (!enc) { set_last_error(__FILE__, __LINE__, "cuTensorMapEncodeTiled unavailable"); return false; }
   cuuint64_t dims[4] = {(cuuint64_t)d, (cuuint64_t)s, (cuuint64_t)h, (cuuint64_t)b};
   cuuint64_t strides[3] = {(cuuint64_t)ss * 2, (cuuint64_t)sh * 2, (cuuint64_t)sb * 2};
   cuuint32_t box[4] = {64, 128, 1, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = enc(out, dtype == kBF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(ptr),
-                   dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_last_error(__FILE__, __LINE__, ("cuTensorMapEncodeTiled (attention bwd) failed: " + std::to_string((int)r)).c_str());
-    return false;
-  }
-  return true;
-}
-static uint32_t make_idesc(int dtype, bool a_mn, bool b_mn) {
-  uint32_t d = 0;
-  d |= 1u << 4;
-  const uint32_t f = dtype == kBF16 ? 1u : 0u;
-  d |= f << 7;
-  d |= f << 10;
-  d |= (a_mn ? 1u : 0u) << 15;
-  d |= (b_mn ? 1u : 0u) << 16;
-  d |= (uint32_t)(128 >> 3) << 17;
-  d |= (uint32_t)(128 >> 4) << 24;
-  return d;
+  return encode_tiled(out, dtype == kBF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, ptr, dims, strides, box,
+                      "attention bwd");
 }
 
 }  // namespace attn_bwd
@@ -421,9 +376,10 @@ int attention_bwd(const AttnBwdArgs& a, cudaStream_t s) {
   p.lse = f.lse; p.delta = a.delta; p.dq = a.dq; p.dk = a.dk; p.dv = a.dv;
   p.dkv_sb = a.dkv_strides[0]; p.dkv_ss = a.dkv_strides[1]; p.dkv_sh = a.dkv_strides[2];
   p.dq_sb = a.dq_strides[0]; p.dq_ss = a.dq_strides[1]; p.dq_sh = a.dq_strides[2];
-  p.idesc_kk = make_idesc(f.dtype, false, false);
-  p.idesc_mm = make_idesc(f.dtype, true, true);
-  p.idesc_mk = make_idesc(f.dtype, true, false);
+  const uint32_t fmt = f.dtype == kBF16 ? 1u : 0u;
+  p.idesc_kk = umma_idesc(fmt, fmt, false, false, BM, BN, false);
+  p.idesc_mm = umma_idesc(fmt, fmt, true, true, BM, BN, false);
+  p.idesc_mk = umma_idesc(fmt, fmt, true, false, BM, BN, false);
   dim3 grid((f.sk + BN - 1) / BN, f.hk, f.b);
   static bool attr_set[4] = {false, false, false, false};
   auto go = [&](auto kern, int slot) {

@@ -17,11 +17,11 @@
 // TMEM columns: [0,128) S stream 0, [128,256) S stream 1, [256,384) O stream 0, [384,512) O stream 1.
 #include <cuda.h>
 #include <cstdio>
-#include <string>
 
 #include "include/b200_common.cuh"
 #include "include/b200_ops.h"
 #include "include/b200_ptx.cuh"
+#include "include/b200_tcgen05_host.h"
 
 namespace b200 {
 namespace attn {
@@ -34,18 +34,6 @@ constexpr uint32_t HALF_BYTES = TILE_BYTES / 2;  // one 64-wide K-block of a til
 constexpr uint32_t SMEM_BYTES = 7 * TILE_BYTES + 1024 /*align*/ + 256 /*barriers*/;   // Q, 2x K, 2x V, 2x P (the epilogue exchange reuses the Q tile)
 constexpr uint32_t TMEM_COLS = 512;
 constexpr uint32_t O_COL = 256;
-
-
-
-template <typename T> __device__ __forceinline__ uint32_t pack2(float a, float b);
-template <> __device__ __forceinline__ uint32_t pack2<__nv_bfloat16>(float a, float b) {
-  const __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<const uint32_t*>(&v);
-}
-template <> __device__ __forceinline__ uint32_t pack2<__half>(float a, float b) {
-  const __half2 v = __floats2half2_rn(a, b);
-  return *reinterpret_cast<const uint32_t*>(&v);
-}
 
 struct Params {
   int b, sq, sk, h, hk;
@@ -97,9 +85,9 @@ fwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CU
   }
 
   if (warp == 8 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_q) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_k) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_v) : "memory");
+    tma_prefetch_desc(&map_q);
+    tma_prefetch_desc(&map_k);
+    tma_prefetch_desc(&map_v);
     mbar_init(q_full, 1);
     for (int s = 0; s < 2; ++s) {
       mbar_init(k_full(s), 1); mbar_init(v_full(s), 1); mbar_init(k_empty(s), 1); mbar_init(v_empty(s), 1);
@@ -110,8 +98,7 @@ fwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CU
     fence_barrier_init();
     fence_proxy_async();
   } else if (warp == 9) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_ptr)), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(smem_u32((const void*)tmem_ptr), TMEM_COLS);
   }
   tc_fence_before();
   __syncthreads();
@@ -270,7 +257,7 @@ fwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CU
           u[e] = pack2<T>(p0, p1);          // one cvt.rn.{bf16x2,f16x2}.f32 per pair
         }
         const uint32_t addr = sP(w) + (c >> 3) * HALF_BYTES + rl * 128 + (((c & 7) ^ (rl & 7)) << 4);
-        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(u[0]), "r"(u[1]), "r"(u[2]), "r"(u[3]) : "memory");
+        st_shared_v4(addr, u[0], u[1], u[2], u[3]);
       }
       l_i += ((sump[0] + sump[1]) + (sump[2] + sump[3])) + ((sump[4] + sump[5]) + (sump[6] + sump[7]));
       fence_proxy_async();     // generic-proxy smem writes -> visible to the tensor core (async proxy)
@@ -338,54 +325,18 @@ fwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CU
   __syncthreads();
   if (warp == 9) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    tmem_dealloc(tmem_base, TMEM_COLS);
   }
 }
 
 // ---------------------------------------------------------------------------------------------- host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)p;
-  }
-  return fn;
-}
-
 // 4-D map {d, s, h, b} over a strided [B,S,H,D] view (strides in elements), box {64, rows, 1, 1}, 128B swizzle
 static bool make_map4(CUtensorMap* out, const void* ptr, int d, int s, int h, int b, int64_t ss, int64_t sh, int64_t sb, uint32_t box_rows, int dtype) {
-  bind_primary_context();
-  EncodeTiledFn enc = get_encode();
-  if (!enc) { set_last_error(__FILE__, __LINE__, "cuTensorMapEncodeTiled unavailable"); return false; }
   cuuint64_t dims[4] = {(cuuint64_t)d, (cuuint64_t)s, (cuuint64_t)h, (cuuint64_t)b};
   cuuint64_t strides[3] = {(cuuint64_t)ss * 2, (cuuint64_t)sh * 2, (cuuint64_t)sb * 2};
   cuuint32_t box[4] = {64, box_rows, 1, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = enc(out, dtype == kBF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(ptr),
-                   dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_last_error(__FILE__, __LINE__, ("cuTensorMapEncodeTiled (attention) failed: " + std::to_string((int)r)).c_str());
-    return false;
-  }
-  return true;
-}
-
-static uint32_t make_idesc(int dtype, int n, bool b_mn) {
-  uint32_t d = 0;
-  d |= 1u << 4;                                  // fp32 accumulate
-  const uint32_t f = dtype == kBF16 ? 1u : 0u;
-  d |= f << 7;
-  d |= f << 10;
-  d |= (b_mn ? 1u : 0u) << 16;                   // B operand MN-major (V: head_dim contiguous)
-  d |= (uint32_t)(n >> 3) << 17;
-  d |= (uint32_t)(BM >> 4) << 24;
-  return d;
+  return encode_tiled(out, dtype == kBF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, ptr, dims, strides, box,
+                      "attention");
 }
 
 }  // namespace attn
@@ -417,8 +368,9 @@ int attention_fwd(const AttnArgs& a, cudaStream_t s) {
   p.o = a.o; p.lse = a.lse;
   p.o_sb = a.o_strides[0]; p.o_ss = a.o_strides[1]; p.o_sh = a.o_strides[2];
   p.dtype = a.dtype;
-  p.idesc_qk = make_idesc(a.dtype, BN, false);
-  p.idesc_pv = make_idesc(a.dtype, HD, true);
+  const uint32_t f = a.dtype == kBF16 ? 1u : 0u;
+  p.idesc_qk = umma_idesc(f, f, false, false, BM, BN, false);
+  p.idesc_pv = umma_idesc(f, f, false, true, BM, HD, false);   // B operand MN-major (V: head_dim contiguous)
   p.colmask = reinterpret_cast<const int4*>(a.colmask);
   p.mask_heads = a.mask_heads > 0 ? a.mask_heads : 1;
   dim3 grid((a.sq + BM - 1) / BM, a.h, a.b);

@@ -8,8 +8,8 @@
 //   all-gather      the multimem.st half: every rank broadcasts its chunk into slot `rank` of every replica.
 //
 // Memory plumbing (multicast object, binding, handle exchange) is torch.distributed._symmetric_memory's; the kernels get the multicast
-// pointer, the local replica pointer and every rank's signal pad.  Cross-rank barriers are the epoch protocol of p2p_collectives.cu on
-// two words at the END of the signal pads (the front belongs to torch's own barrier channels).
+// pointer, the local replica pointer and every rank's signal pad.  Cross-rank barriers are the epoch protocol of the p2p collectives
+// (include/b200_signal_pad.cuh) on two slots at the END of the signal pads (the front belongs to torch's own barrier channels).
 //
 // Status: compiled for sm_100a (SASS holds the multimem instructions); NOT yet run on hardware - opt-in behind FLAGS_b200_nvls.
 // Parity (role): NCCL's NVLS algorithm under ProcessGroupNCCL::AllReduce (paddle/fluid/distributed/collective/process_group_nccl.cc).
@@ -17,6 +17,7 @@
 
 #include "../include/b200_common.cuh"
 #include "../include/b200_comm.h"
+#include "../include/b200_signal_pad.cuh"
 
 namespace b200 {
 namespace comm {
@@ -24,6 +25,7 @@ namespace comm {
 namespace {
 constexpr int kMaxRanks = 8;
 constexpr int kThreads = 512;
+constexpr uint64_t kBarrierTimeoutNs = 10000000000ull;   // 10 s: a dead peer or a protocol bug traps instead of hanging the GPU
 
 struct NvlsPeers {
   uint32_t* pad[kMaxRanks];      // our two barrier rows inside every rank's signal pad: pad[r][slot * kMaxRanks + src]
@@ -31,50 +33,13 @@ struct NvlsPeers {
   char* local;                   // this rank's replica
 };
 
-__device__ __forceinline__ void st_release_sys(uint32_t* p, uint32_t v) {
-  asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ uint32_t ld_acquire_sys(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ uint64_t gtimer() {
-  uint64_t t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-
 __device__ __forceinline__ void signal_all(const NvlsPeers& P, int rank, int world, int slot, uint32_t epoch) {
-  if ((int)threadIdx.x < world && (int)threadIdx.x != rank) st_release_sys(P.pad[threadIdx.x] + slot * kMaxRanks + rank, epoch);
+  pad::signal_all(P.pad, rank, world, slot, epoch);
 }
-
 __device__ __forceinline__ void wait_all(const NvlsPeers& P, int rank, int world, int slot, uint32_t epoch) {
-  if ((int)threadIdx.x < world && (int)threadIdx.x != rank) {
-    const uint32_t* f = P.pad[rank] + slot * kMaxRanks + threadIdx.x;
-    const uint64_t t0 = gtimer();
-    while ((int32_t)(ld_acquire_sys(f) - epoch) < 0) {
-      if (gtimer() - t0 > 10000000000ull) {      // 10 s: fail loudly instead of hanging the GPU
-        printf("b200 nvls: barrier timeout rank %d waiting for %d slot %d epoch %u (have %u)\n", rank, (int)threadIdx.x, slot, epoch, ld_acquire_sys(f));
-        __trap();
-      }
-    }
-  }
-  __syncthreads();
+  pad::wait_all(P.pad, rank, world, slot, epoch, kBarrierTimeoutNs, B200_PAD_TIMEOUT("nvls"));
 }
-
-__device__ __forceinline__ bool last_cta(uint32_t* counter) {
-  __shared__ bool is_last;
-  __threadfence_system();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const uint32_t prev = atomicAdd(counter, 1u);
-    is_last = (prev == gridDim.x - 1);
-    if (is_last) *counter = 0;
-  }
-  __syncthreads();
-  return is_last;
-}
+using pad::last_cta;
 
 // 16 bytes reduced across every replica by the switch (fp32 accumulation for the 16-bit types)
 template <typename T> struct Mm;

@@ -14,69 +14,28 @@
 
 #include "../include/b200_common.cuh"
 #include "../include/b200_comm.h"
+#include "../include/b200_signal_pad.cuh"
 
 namespace b200 {
 namespace comm {
 
 constexpr int kMaxRanks = 8;
 constexpr int kThreads = 512;
+constexpr uint64_t kBarrierTimeoutNs = 10000000000ull;   // 10 s: a dead peer or a protocol bug traps instead of hanging the GPU
 
 struct Peers {
   char* base[kMaxRanks];
 };
 
-__device__ __forceinline__ void st_release_sys(uint32_t* p, uint32_t v) {
-  asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ uint32_t ld_acquire_sys(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ uint64_t gtimer() {
-  uint64_t t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-
-// pad layout: uint32 pad[kSlots][kMaxRanks] at heap base
-__device__ __forceinline__ uint32_t* pad_ptr(char* base, int slot, int src) {
-  return reinterpret_cast<uint32_t*>(base) + slot * kMaxRanks + src;
-}
-
-// All threads of the CTA return once every peer has published `epoch` in local pad[slot].
-__device__ __forceinline__ void wait_all(const Peers& P, int rank, int world, int slot, uint32_t epoch) {
-  if ((int)threadIdx.x < world && (int)threadIdx.x != rank) {
-    const uint32_t* f = pad_ptr(P.base[rank], slot, threadIdx.x);
-    const uint64_t t0 = gtimer();
-    // epochs are monotonically increasing; signed distance handles wrap-around
-    while ((int32_t)(ld_acquire_sys(f) - epoch) < 0) {
-      if (gtimer() - t0 > 10000000000ull) {  // 10 s: peer died or protocol bug -> fail loudly, do not hang the GPU
-        printf("b200 p2p: barrier timeout rank %d waiting for %d slot %d epoch %u (have %u)\n", rank, (int)threadIdx.x, slot, epoch, ld_acquire_sys(f));
-        __trap();
-      }
-    }
-  }
-  __syncthreads();
-}
-
+// the signal pad of every rank is the first bytes of its heap slab
+__device__ __forceinline__ uint32_t* const* pads(const Peers& P) { return reinterpret_cast<uint32_t* const*>(P.base); }
 __device__ __forceinline__ void signal_all(const Peers& P, int rank, int world, int slot, uint32_t epoch) {
-  if ((int)threadIdx.x < world && (int)threadIdx.x != rank) st_release_sys(pad_ptr(P.base[threadIdx.x], slot, rank), epoch);
+  pad::signal_all(pads(P), rank, world, slot, epoch);
 }
-
-// Grid-wide completion: returns true in the last CTA to arrive.
-__device__ __forceinline__ bool last_cta(uint32_t* counter) {
-  __shared__ bool is_last;
-  __threadfence_system();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const uint32_t prev = atomicAdd(counter, 1u);
-    is_last = (prev == gridDim.x - 1);
-    if (is_last) *counter = 0;  // reset for the next launch (stream-ordered)
-  }
-  __syncthreads();
-  return is_last;
+__device__ __forceinline__ void wait_all(const Peers& P, int rank, int world, int slot, uint32_t epoch) {
+  pad::wait_all(pads(P), rank, world, slot, epoch, kBarrierTimeoutNs, B200_PAD_TIMEOUT("p2p"));
 }
+using pad::last_cta;
 
 // ---------------------------------------------------------------------------------------------- two-shot all-reduce
 // buffer of n elements at `off` in every rank's heap. Rank r owns elements [r*chunk, (r+1)*chunk): it reads that range
@@ -366,20 +325,20 @@ void p2p_gather_pull(const int64_t* bases, int64_t src_off, void* dst, int64_t c
 // slot.  The waiting thread accounts the time it spun into stats[0] (ns) / stats[1] (waits) = exposed pipeline wait on the device.
 __global__ void signal_flag_kernel(uint32_t* remote_flag, uint32_t value) {
   __threadfence_system();
-  st_release_sys(remote_flag, value);
+  ptx::st_release_sys_u32(remote_flag, value);
 }
 
 __global__ void wait_flag_kernel(const uint32_t* flag, uint32_t value, unsigned long long* stats, unsigned long long timeout_ns) {
-  const uint64_t t0 = gtimer();
-  while ((int32_t)(ld_acquire_sys(flag) - value) < 0) {
-    if (gtimer() - t0 > timeout_ns) {
-      printf("b200 p2p mailbox: timeout waiting for flag value %u (have %u)\n", value, ld_acquire_sys(flag));
+  const uint64_t t0 = ptx::globaltimer_ns();
+  while ((int32_t)(ptx::ld_acquire_sys_u32(flag) - value) < 0) {
+    if (ptx::globaltimer_ns() - t0 > timeout_ns) {
+      printf("b200 p2p mailbox: timeout waiting for flag value %u (have %u)\n", value, ptx::ld_acquire_sys_u32(flag));
       __trap();
     }
     __nanosleep(200);
   }
   if (stats) {
-    atomicAdd(stats, (unsigned long long)(gtimer() - t0));
+    atomicAdd(stats, (unsigned long long)(ptx::globaltimer_ns() - t0));
     atomicAdd(stats + 1, 1ull);
   }
 }

@@ -12,12 +12,11 @@
 // Parity (behaviour): fp8_fp8_half_gemm_fused (paddle/phi/kernels/fusion/fp8_gemm/fp8_gemm_with_cublasLt/*) which calls cuBLASLt.
 #include <cuda.h>
 #include <cstdio>
-#include <cstdlib>
-#include <string>
 
 #include "include/b200_common.cuh"
 #include "include/b200_ops.h"
 #include "include/b200_ptx.cuh"
+#include "include/b200_tcgen05_host.h"
 
 namespace b200 {
 namespace gemm8 {
@@ -51,12 +50,6 @@ template <int BN, bool MX = false> struct Cfg {
   static_assert(SMEM_BYTES <= 232448, "fp8 gemm: shared memory budget");
 };
 
-
-
-
-
-
-
 struct Params {
   int m, n, k, batch;
   void* d;
@@ -71,32 +64,6 @@ struct Params {
   const uint8_t* sfb;
   uint32_t idesc;
 };
-
-__device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.f + erff(x * 0.70710678118654752f)); }
-
-template <typename TO>
-__device__ __forceinline__ void store_row_chunk(TO* __restrict__ dst, const float (&v)[32], int valid, bool accumulate) {
-  if (valid >= 32 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
-    constexpr int N = Vec16<TO>::N;
-#pragma unroll
-    for (int q = 0; q < 32 / N; ++q) {
-      Vec16<TO> o;
-      if (accumulate) {
-        Vec16<TO> old = ld16(dst + q * N);
-#pragma unroll
-        for (int j = 0; j < N; ++j) o.v[j] = from_f<TO>(v[q * N + j] + to_f(old.v[j]));
-      } else {
-#pragma unroll
-        for (int j = 0; j < N; ++j) o.v[j] = from_f<TO>(v[q * N + j]);
-      }
-      st16(dst + q * N, o);
-    }
-  } else {
-#pragma unroll
-    for (int j = 0; j < 32; ++j)
-      if (j < valid) dst[j] = from_f<TO>(accumulate ? v[j] + to_f(dst[j]) : v[j]);
-  }
-}
 
 template <int BN, bool MX>
 __global__ void __launch_bounds__(kThreads, 1)
@@ -126,8 +93,7 @@ gemm_fp8_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
     fence_barrier_init();
     fence_proxy_async();
   } else if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_ptr_smem)), "r"(C::TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(smem_u32((const void*)tmem_ptr_smem), C::TMEM_COLS);
   }
   tc_fence_before();
   __syncthreads();
@@ -283,61 +249,17 @@ gemm_fp8_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
   __syncthreads();
   if (warp == 2) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(C::TMEM_COLS) : "memory");
+    tmem_dealloc(tmem_base, C::TMEM_COLS);
   }
 }
 
 // ---------------------------------------------------------------------------------------------- host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)p;
-  }
-  return fn;
-}
 // 3-D byte map {k (contiguous), rows, batch}
 static bool make_map8(CUtensorMap* out, const void* ptr, uint64_t k, uint64_t rows, uint64_t batch, uint64_t ld, uint64_t bstride, uint32_t box_rows) {
-  bind_primary_context();
-  EncodeTiledFn enc = get_encode();
-  if (!enc) { set_last_error(__FILE__, __LINE__, "cuTensorMapEncodeTiled unavailable"); return false; }
   cuuint64_t dims[3] = {k, rows, batch};
   cuuint64_t strides[2] = {ld, batch > 1 ? bstride : rows * ld};
   cuuint32_t box[3] = {(cuuint32_t)BLOCK_K, box_rows, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_last_error(__FILE__, __LINE__, ("cuTensorMapEncodeTiled (fp8) failed: " + std::to_string((int)r)).c_str());
-    return false;
-  }
-  return true;
-}
-static uint32_t make_idesc(int a_e5m2, int b_e5m2, int bn) {
-  uint32_t d = 0;
-  d |= 1u << 4;                                   // c_format = F32
-  d |= (a_e5m2 ? 1u : 0u) << 7;                   // a_format: E4M3 = 0, E5M2 = 1
-  d |= (b_e5m2 ? 1u : 0u) << 10;                  // b_format
-  d |= (uint32_t)(bn >> 3) << 17;                 // n_dim
-  d |= (uint32_t)(BLOCK_M >> 4) << 24;            // m_dim
-  return d;
-}
-
-// block-scaled descriptor (cute::UMMA::InstrDescriptorBlockScaled): no c_format (always fp32); bits [4,6) b_sf_id, 23 scale format
-// (1 = E8M0), [29,31) a_sf_id - the two ids are OR-ed in per MMA
-static uint32_t make_idesc_mx(int a_e5m2, int b_e5m2, int bn) {
-  uint32_t d = 0;
-  d |= (a_e5m2 ? 1u : 0u) << 7;
-  d |= (b_e5m2 ? 1u : 0u) << 10;
-  d |= (uint32_t)(bn >> 3) << 17;
-  d |= 1u << 23;
-  d |= (uint32_t)(BLOCK_M >> 4) << 24;
-  return d;
+  return encode_tiled(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, ptr, dims, strides, box, "fp8 gemm");
 }
 
 template <int BN, bool MX>
@@ -357,7 +279,7 @@ static int launch(const GemmFp8Args& g, cudaStream_t s) {
   p.scale = g.scale;
   p.scale_a = g.scale_a_dev; p.scale_b = g.scale_b_dev;
   p.sfa = g.sfa; p.sfb = g.sfb;
-  p.idesc = MX ? make_idesc_mx(g.a_e5m2, g.b_e5m2, BN) : make_idesc(g.a_e5m2, g.b_e5m2, BN);
+  p.idesc = umma_idesc(g.a_e5m2 ? 1u : 0u, g.b_e5m2 ? 1u : 0u, false, false, BLOCK_M, BN, MX);   // E4M3 = 0, E5M2 = 1
   static bool attr_set = false;
   auto kern = gemm_fp8_kernel<BN, MX>;
   if (!attr_set) {

@@ -11,14 +11,13 @@
 // Warp roles (256 threads): w0 TMA producer | w1 MMA issuer | w2 TMEM allocator | w4..w7 epilogue (TMEM lane quadrants).
 #include <cuda.h>
 #include <cstdio>
-#include <cstdlib>
 #include <mutex>
 #include <unordered_map>
-#include <string>
 
 #include "include/b200_common.cuh"
 #include "include/b200_ops.h"
 #include "include/b200_ptx.cuh"
+#include "include/b200_tcgen05_host.h"
 
 namespace b200 {
 namespace gemm {
@@ -39,12 +38,6 @@ template <int BN> struct Cfg {
   static constexpr uint32_t SMEM_BYTES = kStages * STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/;
 };
 
-
-
-
-
-
-
 struct Params {
   int m, n, k, batch;
   void* d;
@@ -56,32 +49,6 @@ struct Params {
   int rs_world, rs_rows;   // fused reduce-scatter push (see GemmArgs)
   void* rs_dst[8];
 };
-
-__device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.f + erff(x * 0.70710678118654752f)); }
-
-template <typename TO>
-__device__ __forceinline__ void store_row_chunk(TO* __restrict__ dst, const float (&v)[32], int valid, bool accumulate) {
-  if (valid >= 32 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
-    constexpr int N = Vec16<TO>::N;
-#pragma unroll
-    for (int q = 0; q < 32 / N; ++q) {
-      Vec16<TO> o;
-      if (accumulate) {
-        Vec16<TO> old = ld16(dst + q * N);
-#pragma unroll
-        for (int j = 0; j < N; ++j) o.v[j] = from_f<TO>(v[q * N + j] + to_f(old.v[j]));
-      } else {
-#pragma unroll
-        for (int j = 0; j < N; ++j) o.v[j] = from_f<TO>(v[q * N + j]);
-      }
-      st16(dst + q * N, o);
-    }
-  } else {
-#pragma unroll
-    for (int j = 0; j < 32; ++j)
-      if (j < valid) dst[j] = from_f<TO>(accumulate ? v[j] + to_f(dst[j]) : v[j]);
-  }
-}
 
 template <int BN, bool A_MN, bool B_MN>
 __global__ void __launch_bounds__(kThreads, 1)
@@ -111,8 +78,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ C
     fence_barrier_init();
     fence_proxy_async();
   } else if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_ptr_smem)), "r"(C::TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(smem_u32((const void*)tmem_ptr_smem), C::TMEM_COLS);
   }
   tc_fence_before();
   __syncthreads();
@@ -266,26 +232,11 @@ gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ C
   __syncthreads();
   if (warp == 2) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(C::TMEM_COLS) : "memory");
+    tmem_dealloc(tmem_base, C::TMEM_COLS);
   }
 }
 
 // ---------------------------------------------------------------------------------------------- host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)p;
-  }
-  return fn;
-}
-
 struct MapKey {
   const void* ptr; uint64_t inner, rows, batch, ld, bstride; uint32_t box_inner, box_rows; int dtype;
   bool operator==(const MapKey& o) const {
@@ -302,9 +253,8 @@ struct MapKeyHash {
   }
 };
 
-// 3-D map {inner (contiguous), rows, batch}; element = 2 bytes (bf16 / fp16) or 4 bytes (kF32: TMA-store maps of fp32 outputs).
-bool make_map(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t rows, uint64_t batch, uint64_t ld,
-                     uint64_t bstride, uint32_t box_inner, uint32_t box_rows, int dtype) {
+bool make_map(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t rows, uint64_t batch, uint64_t ld, uint64_t bstride,
+              uint32_t box_inner, uint32_t box_rows, int dtype) {
   static std::mutex mu;
   static std::unordered_map<MapKey, CUtensorMap, MapKeyHash> cache;
   MapKey key{ptr, inner, rows, batch, ld, bstride, box_inner, box_rows, dtype};
@@ -313,38 +263,17 @@ bool make_map(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t rows, 
     auto it = cache.find(key);
     if (it != cache.end()) { *out = it->second; return true; }
   }
-  bind_primary_context();
-  EncodeTiledFn enc = get_encode();
-  if (!enc) { set_last_error(__FILE__, __LINE__, "cuTensorMapEncodeTiled unavailable"); return false; }
   cuuint64_t dims[3] = {inner, rows, batch};
   const uint64_t es = dtype == kF32 ? 4 : 2;
   cuuint64_t strides[2] = {ld * es, (batch > 1 ? bstride : rows * ld) * es};
   cuuint32_t box[3] = {box_inner, box_rows, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(out, dtype == kBF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : (dtype == kF32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16), 3,
-                   const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_last_error(__FILE__, __LINE__, ("cuTensorMapEncodeTiled failed: " + std::to_string((int)r)).c_str());
-    return false;
-  }
+  const CUtensorMapDataType type =
+      dtype == kBF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : (dtype == kF32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16);
+  if (!encode_tiled(out, type, 3, ptr, dims, strides, box, "gemm")) return false;
   std::lock_guard<std::mutex> g(mu);
   if (cache.size() > 8192) cache.clear();
   cache.emplace(key, *out);
   return true;
-}
-
-static uint32_t make_idesc(int in_dtype, int bn, bool a_mn, bool b_mn) {
-  uint32_t d = 0;
-  d |= 1u << 4;                                   // c_format = F32
-  const uint32_t f = in_dtype == kBF16 ? 1u : 0u; // F16 = 0, BF16 = 1
-  d |= f << 7;                                    // a_format
-  d |= f << 10;                                   // b_format
-  d |= (a_mn ? 1u : 0u) << 15;                    // a_major (1 = MN-major)
-  d |= (b_mn ? 1u : 0u) << 16;                    // b_major
-  d |= (uint32_t)(bn >> 3) << 17;                 // n_dim
-  d |= (uint32_t)(BLOCK_M >> 4) << 24;            // m_dim
-  return d;
 }
 
 template <int BN, bool A_MN, bool B_MN>
@@ -370,7 +299,8 @@ static int launch(const GemmArgs& g, cudaStream_t s) {
   p.rs_rows = g.rs_rows;
   for (int i = 0; i < 8; ++i) p.rs_dst[i] = g.rs_dst[i];
   if (p.rs_world) p.ldd = g.n;
-  p.idesc = make_idesc(g.dtype, BN, A_MN, B_MN);
+  const uint32_t f = g.dtype == kBF16 ? 1u : 0u;
+  p.idesc = umma_idesc(f, f, A_MN, B_MN, BLOCK_M, BN, false);
   static bool attr_set = false;
   auto kern = gemm_kernel<BN, A_MN, B_MN>;
   if (!attr_set) {
@@ -407,10 +337,9 @@ int gemm_tcgen05(const GemmArgs& g, cudaStream_t s) {
   if (!gemm_tcgen05_supported(g.m, g.n, g.k, g.lda, g.ldb, g.ldd, g.a_is_km, g.b_is_nk)) return 1;
   if ((reinterpret_cast<uintptr_t>(g.a) & 15) || (reinterpret_cast<uintptr_t>(g.b) & 15)) return 1;
   if (g.dtype != kBF16 && g.dtype != kF16) return 1;
-  // large problems: CTA-pair kernel (cta_group::2, 256x256 cluster tile); B200_GEMM_2CTA=0 forces the 1-CTA kernel
-  static const int use_2cta = [] { const char* e = getenv("B200_GEMM_2CTA"); return e ? atoi(e) : 1; }();
   if (g.ag_world > 1) return gemm_tcgen05_2cta(g, s);   // the fused all-gather lives in the CTA-pair kernel only
-  if (use_2cta && g.m >= 256 && g.n >= 256) return gemm_tcgen05_2cta(g, s);
+  // large problems: CTA-pair kernel (cta_group::2, 256x256 cluster tile)
+  if (g.m >= 256 && g.n >= 256) return gemm_tcgen05_2cta(g, s);
   // tile-N choice: widest tile that keeps the last wave reasonably full
   const int sms = sm_count();
   auto waves_eff = [&](int bn) {

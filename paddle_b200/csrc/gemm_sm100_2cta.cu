@@ -18,12 +18,9 @@
 #include "include/b200_common.cuh"
 #include "include/b200_ops.h"
 #include "include/b200_ptx.cuh"
+#include "include/b200_tcgen05_host.h"
 
 namespace b200 {
-namespace gemm {
-bool make_map(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t rows, uint64_t batch, uint64_t ld, uint64_t bstride,
-              uint32_t box_inner, uint32_t box_rows, int dtype);
-}
 namespace gemm2 {
 using namespace ptx;
 
@@ -44,76 +41,12 @@ constexpr uint32_t STG_BOX_BYTES = 32 * 128;
 constexpr uint32_t STG_OFF = kStages * STAGE_BYTES + 1024;                 // after the barrier page (1024-aligned)
 constexpr uint32_t STG_BYTES = 4 * 2 * STG_BOX_BYTES;                      // 32 KB
 constexpr uint32_t SMEM_BYTES = STG_OFF + STG_BYTES + 1024;                // + alignment slack = 231424 <= 232448 (227 KB)
-constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;              // clears the CTA-rank bit of a shared::cluster address
-
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-// arrive on the barrier at the same smem offset in cluster CTA `rank`
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar, uint32_t rank) {
-  asm volatile(
-      "{\n\t.reg .b32 ra;\n\t"
-      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-      "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}"
-      ::"r"(bar), "r"(rank)
-      : "memory");
-}
-
-// TMA load whose completion bytes are credited to the LEADER CTA's mbarrier
-__device__ __forceinline__ void tma_load_3d_2sm(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, int c2, uint64_t hint) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
-      " [%0], [%1, {%3, %4, %5}], [%2], %6;"
-      ::"r"(dst), "l"(map), "r"(bar & kPeerBitMask), "r"(c0), "r"(c1), "r"(c2), "l"(hint)
-      : "memory");
-}
-// smem box -> global (or peer) memory; completion tracked by the issuing thread's bulk async-group
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, uint32_t src, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-               ::"l"(map), "r"(src), "r"(c0), "r"(c1), "r"(c2)
-               : "memory");
-}
-// same box, but added to the destination (bf16 / fp16 / fp32 add performed by the L2 reduction units): D += tile without reading D
-__device__ __forceinline__ void tma_reduce_add_3d(const CUtensorMap* map, uint32_t src, int c0, int c1, int c2) {
-  asm volatile("cp.reduce.async.bulk.tensor.3d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3, %4}], [%1];"
-               ::"l"(map), "r"(src), "r"(c0), "r"(c1), "r"(c2)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read_1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-__device__ __forceinline__ uint32_t pack2_bf16(float a, float b) {
-  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
-__device__ __forceinline__ uint32_t pack2_f16(float a, float b) {
-  __half2 h = __floats2half2_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
-__device__ __forceinline__ void umma_f16_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// commit -> arrive on the barrier at this offset in BOTH CTAs of the pair
-__device__ __forceinline__ void umma_commit_2sm(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"((uint16_t)0x3)
-               : "memory");
-}
 
 struct DMaps { CUtensorMap m[8]; };   // TMA-store maps of the output: [0] = D, or one per reduce-scatter owner slot
 
 struct Params {
-  int tma_store;           // epilogue goes TMEM -> registers -> swizzled smem -> cp.async.bulk.tensor (UTMASTG), also to peer HBM
+  int tma_store;           // epilogue goes TMEM -> registers -> swizzled smem -> cp.async.bulk.tensor (UTMASTG), also to peer HBM;
+                           // 0: registers -> global stores (output rows that are not 16-byte aligned)
   int m, n, k, batch;
   void* d;
   const void* bias;
@@ -140,30 +73,15 @@ struct Params {
 constexpr int kAgChunkBytes = 16384;
 constexpr int kAgReadySlot = 4, kAgDoneSlot = 5, kPadRanks = 8;
 
-__device__ __forceinline__ void st_release_sys_u32(uint32_t* p, uint32_t v) {
-  asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+// the all-gather's cross-rank waits; a peer that stalls traps with a message naming this protocol
+__device__ __forceinline__ void ag_wait(const uint32_t* p, uint32_t epoch, const char* what) {
+  spin_sys_ge(p, epoch, "b200 gemm2 all-gather: timeout waiting for %s\n", what);
 }
-__device__ __forceinline__ uint32_t ld_acquire_sys_u32(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ uint32_t ld_acquire_gpu_u32(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-// bounded spins: a dead peer / protocol bug traps instead of hanging the GPU
-__device__ __forceinline__ void spin_sys_ge(const uint32_t* p, uint32_t target, const char* what) {
-  const uint64_t t0 = globaltimer_ns();
-  while ((int32_t)(ld_acquire_sys_u32(p) - target) < 0) {
-    if (globaltimer_ns() - t0 > 10000000000ull) { printf("b200 gemm2 all-gather: timeout waiting for %s\n", what); __trap(); }
-  }
-}
+// bounded spin on a gathered row block's chunk counter (bumped by the copy warps of this GPU)
 __device__ __forceinline__ void spin_gpu_ge(const uint32_t* p, uint32_t target) {
   const uint64_t t0 = globaltimer_ns();
   while (ld_acquire_gpu_u32(p) < target) {
-    if (globaltimer_ns() - t0 > 10000000000ull) { printf("b200 gemm2 all-gather: timeout waiting for a gathered row block\n"); __trap(); }
+    if (globaltimer_ns() - t0 > kSpinTimeoutNs) { printf("b200 gemm2 all-gather: timeout waiting for a gathered row block\n"); __trap(); }
   }
 }
 
@@ -185,7 +103,7 @@ __device__ __forceinline__ void ag_copy_role(const Params& p, int lane) {
     const int64_t rem = g - (int64_t)(pr - 1) * per_src;
     const int blk_in = (int)(rem / p.ag_chunks), ch = (int)(rem % p.ag_chunks);
     if (src != cur_src) {
-      if (lane == 0) spin_sys_ge(my_pad + kAgReadySlot * kPadRanks + src, p.ag_epoch, "a peer shard");
+      if (lane == 0) ag_wait(my_pad + kAgReadySlot * kPadRanks + src, p.ag_epoch, "a peer shard");
       __syncwarp();
       cur_src = src;
     }
@@ -215,33 +133,7 @@ __device__ __forceinline__ void ag_copy_role(const Params& p, int lane) {
     }
   }
   if (wid == 0 && lane < p.ag_world && lane != p.ag_rank)        // peers finished reading my shard: it may be reused after exit
-    spin_sys_ge(my_pad + kAgDoneSlot * kPadRanks + lane, p.ag_epoch, "a peer to finish reading");
-}
-
-__device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.f + erff(x * 0.70710678118654752f)); }
-
-template <typename TO>
-__device__ __forceinline__ void store_row_chunk(TO* __restrict__ dst, const float (&v)[32], int valid, bool accumulate) {
-  if (valid >= 32 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
-    constexpr int N = Vec16<TO>::N;
-#pragma unroll
-    for (int q = 0; q < 32 / N; ++q) {
-      Vec16<TO> o;
-      if (accumulate) {
-        Vec16<TO> old = ld16(dst + q * N);
-#pragma unroll
-        for (int j = 0; j < N; ++j) o.v[j] = from_f<TO>(v[q * N + j] + to_f(old.v[j]));
-      } else {
-#pragma unroll
-        for (int j = 0; j < N; ++j) o.v[j] = from_f<TO>(v[q * N + j]);
-      }
-      st16(dst + q * N, o);
-    }
-  } else {
-#pragma unroll
-    for (int j = 0; j < 32; ++j)
-      if (j < valid) dst[j] = from_f<TO>(accumulate ? v[j] + to_f(dst[j]) : v[j]);
-  }
+    ag_wait(my_pad + kAgDoneSlot * kPadRanks + lane, p.ag_epoch, "a peer to finish reading");
 }
 
 template <bool A_MN, bool B_MN>
@@ -277,8 +169,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
   }
   cluster_sync();  // barriers of both CTAs are initialised before any remote arrive / TMA completion can target them
   if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_ptr_smem)), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    tmem_alloc<2>(smem_u32((const void*)tmem_ptr_smem), TMEM_COLS);
   }
   tc_fence_before();
   __syncthreads();
@@ -429,7 +320,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
         for (int c = 0; c < BLOCK_N / cpb; ++c) {
           const int col0 = nb * BLOCK_N + c * cpb;
           if (col0 >= p.n || row0 >= p.m) break;
-          if (lane == 0) bulk_wait_read_1();        // the box stored two iterations ago has been read out of this buffer
+          if (lane == 0) bulk_wait_read<1>();       // the box stored two iterations ago has been read out of this buffer
           __syncwarp();
           const uint32_t dst = stg + (uint32_t)tma_buf * STG_BOX_BYTES + (uint32_t)lane * 128;
           const uint32_t sw = (uint32_t)(lane & 7);
@@ -468,13 +359,14 @@ gemm2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
             } else if (p.out_dtype == kBF16) {
 #pragma unroll
               for (int q = 0; q < 4; ++q)
-                st_shared_v4(dst + (((uint32_t)(h * 4 + q) ^ sw) << 4), pack2_bf16(v[8 * q], v[8 * q + 1]), pack2_bf16(v[8 * q + 2], v[8 * q + 3]),
-                             pack2_bf16(v[8 * q + 4], v[8 * q + 5]), pack2_bf16(v[8 * q + 6], v[8 * q + 7]));
+                st_shared_v4(dst + (((uint32_t)(h * 4 + q) ^ sw) << 4), pack2<__nv_bfloat16>(v[8 * q], v[8 * q + 1]),
+                             pack2<__nv_bfloat16>(v[8 * q + 2], v[8 * q + 3]), pack2<__nv_bfloat16>(v[8 * q + 4], v[8 * q + 5]),
+                             pack2<__nv_bfloat16>(v[8 * q + 6], v[8 * q + 7]));
             } else {
 #pragma unroll
               for (int q = 0; q < 4; ++q)
-                st_shared_v4(dst + (((uint32_t)(h * 4 + q) ^ sw) << 4), pack2_f16(v[8 * q], v[8 * q + 1]), pack2_f16(v[8 * q + 2], v[8 * q + 3]),
-                             pack2_f16(v[8 * q + 4], v[8 * q + 5]), pack2_f16(v[8 * q + 6], v[8 * q + 7]));
+                st_shared_v4(dst + (((uint32_t)(h * 4 + q) ^ sw) << 4), pack2<__half>(v[8 * q], v[8 * q + 1]), pack2<__half>(v[8 * q + 2], v[8 * q + 3]),
+                             pack2<__half>(v[8 * q + 4], v[8 * q + 5]), pack2<__half>(v[8 * q + 6], v[8 * q + 7]));
             }
           }
           fence_proxy_async();                      // generic-proxy smem writes -> visible to the TMA (async proxy)
@@ -536,28 +428,15 @@ gemm2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(tempty_bar(as), 0);  // leader's barrier counts both CTAs' epilogue warps
     }
-    if (p.tma_store && lane == 0) bulk_wait_all();   // every box has been written before the CTA may exit
+    if (p.tma_store && lane == 0) bulk_wait<0>();    // every box has been written before the CTA may exit
   }
 
   tc_fence_before();
   cluster_sync();  // peer smem / TMEM stay valid until every MMA and remote arrive has retired
   if (warp == 2) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    tmem_dealloc<2>(tmem_base, TMEM_COLS);
   }
-}
-
-static uint32_t make_idesc(int in_dtype, bool a_mn, bool b_mn) {
-  uint32_t d = 0;
-  d |= 1u << 4;
-  const uint32_t f = in_dtype == kBF16 ? 1u : 0u;
-  d |= f << 7;
-  d |= f << 10;
-  d |= (a_mn ? 1u : 0u) << 15;
-  d |= (b_mn ? 1u : 0u) << 16;
-  d |= (uint32_t)(BLOCK_N >> 3) << 17;
-  d |= (uint32_t)((2 * BLOCK_M) >> 4) << 24;   // UMMA M = 256 across the CTA pair
-  return d;
 }
 
 template <bool A_MN, bool B_MN>
@@ -605,27 +484,23 @@ static int launch(const GemmArgs& g, cudaStream_t s) {
   // TMA reduce-add (UTMAREDG): the addition happens in L2 and D is never read by the SMs
   DMaps dm;
   memset(&dm, 0, sizeof(dm));
-  p.tma_store = 0;
   {
     const int es = g.out_dtype == kF32 ? 4 : 2;
     const uint32_t cpb = 128 / es;
-    static const bool enabled = []() { const char* e = getenv("B200_GEMM_TMA_STORE"); return !(e && e[0] == '0'); }();
-    static const bool reduce_ok = []() { const char* e = getenv("B200_GEMM_TMA_REDUCE"); return !(e && e[0] == '0'); }();
-    if (enabled && (!p.accumulate || reduce_ok)) {
-      bool ok2 = true;
-      if (p.rs_world) {
-        ok2 = (g.n * es) % 16 == 0 && g.rs_rows % 32 == 0;
-        for (int r = 0; r < p.rs_world && ok2; ++r)
-          ok2 = ((uintptr_t)g.rs_dst[r] % 16 == 0) && gemm::make_map(&dm.m[r], g.rs_dst[r], g.n, g.rs_rows, 1, g.n, 0, cpb, 32, g.out_dtype);
-      } else {
-        ok2 = (g.ldd * es) % 16 == 0 && ((uintptr_t)g.d % 16 == 0) && (batch == 1 || (g.stride_d * es) % 16 == 0) &&
-              gemm::make_map(&dm.m[0], g.d, g.n, g.m, batch, g.ldd, g.stride_d, cpb, 32, g.out_dtype);
-      }
-      if (!ok2) take_last_error();     // an odd leading dimension just keeps the register-store epilogue
-      p.tma_store = ok2 ? 1 : 0;
+    bool ok2 = true;
+    if (p.rs_world) {
+      ok2 = (g.n * es) % 16 == 0 && g.rs_rows % 32 == 0;
+      for (int r = 0; r < p.rs_world && ok2; ++r)
+        ok2 = ((uintptr_t)g.rs_dst[r] % 16 == 0) && gemm::make_map(&dm.m[r], g.rs_dst[r], g.n, g.rs_rows, 1, g.n, 0, cpb, 32, g.out_dtype);
+    } else {
+      ok2 = (g.ldd * es) % 16 == 0 && ((uintptr_t)g.d % 16 == 0) && (batch == 1 || (g.stride_d * es) % 16 == 0) &&
+            gemm::make_map(&dm.m[0], g.d, g.n, g.m, batch, g.ldd, g.stride_d, cpb, 32, g.out_dtype);
     }
+    if (!ok2) take_last_error();     // an odd leading dimension just keeps the register-store epilogue
+    p.tma_store = ok2 ? 1 : 0;
   }
-  p.idesc = make_idesc(g.dtype, A_MN, B_MN);
+  const uint32_t f = g.dtype == kBF16 ? 1u : 0u;
+  p.idesc = umma_idesc(f, f, A_MN, B_MN, 2 * BLOCK_M, BLOCK_N, false);   // UMMA M = 256 across the CTA pair
   static bool attr_set = false;
   auto kern = gemm2_kernel<A_MN, B_MN>;
   if (!attr_set) {

@@ -13,17 +13,13 @@
 // Parity: paddle/phi/kernels/gpu/weight_only_linear_kernel.cu:27, python/paddle/nn/quant/quantized_linear.py:183.
 #include <cuda.h>
 #include <cstdio>
-#include <string>
 
 #include "include/b200_common.cuh"
 #include "include/b200_ops.h"
 #include "include/b200_ptx.cuh"
+#include "include/b200_tcgen05_host.h"
 
 namespace b200 {
-namespace gemm {
-bool make_map(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t rows, uint64_t batch, uint64_t ld, uint64_t bstride,
-              uint32_t box_inner, uint32_t box_rows, int dtype);
-}
 namespace wo {
 using namespace ptx;
 
@@ -107,8 +103,8 @@ wo_gemm_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
   const int num_kb = max(0, min(p.kb_per_split, num_kb_total - kb0));
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_w) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_x) : "memory");
+    tma_prefetch_desc(&map_w);
+    tma_prefetch_desc(&map_x);
     for (int s = 0; s < WST; ++s) { mbar_init(w_full(s), 1); mbar_init(w_empty(s), KB_PER_W * 4); }
     for (int s = 0; s < XST; ++s) { mbar_init(x_full(s), 1); mbar_init(x_empty(s), 1); }
     for (int s = 0; s < G; ++s) { mbar_init(a_ready(s), 4); mbar_init(a_empty(s), 1); }
@@ -116,8 +112,7 @@ wo_gemm_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
     fence_barrier_init();
     fence_proxy_async();
   } else if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_ptr)), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(smem_u32((const void*)tmem_ptr), TMEM_COLS);
   }
   tc_fence_before();
   __syncthreads();
@@ -305,18 +300,15 @@ wo_gemm_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
     // r, r + splits, ... over all ranks (ld.shared::cluster) and writes the scaled result.  No workspace, no atomics, no second kernel.
     cluster_sync();
     if (warp >= 4 && warp < 8) {
-      uint32_t rank;
-      asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
+      const uint32_t rank = cluster_ctarank();
       const int tok_n = min(NTOK, p.m - tok0);
       for (int c = (int)rank * 4 + (warp - 4); c < tok_n * 4; c += p.splits * 4) {
         const int tok = c >> 2, chl = (c & 3) * 32 + lane, ch = n0 + chl;
         float acc = 0.f;
         const uint32_t local = wring + (uint32_t)((tok * BLOCK_N + chl) * 4);
         for (int q = 0; q < p.splits; ++q) {
-          uint32_t remote;
           float v;
-          asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(local), "r"(q));
-          asm volatile("ld.shared::cluster.f32 %0, [%1];" : "=f"(v) : "r"(remote) : "memory");
+          asm volatile("ld.shared::cluster.f32 %0, [%1];" : "=f"(v) : "r"(mapa(local, q)) : "memory");
           acc += v;
         }
         if (ch < p.n) {
@@ -332,46 +324,16 @@ wo_gemm_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    tmem_dealloc(tmem_base, TMEM_COLS);
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess) fn = (EncodeTiledFn)p;
-  }
-  return fn;
-}
 // raw weights as bytes: [n rows, row_bytes], box {128 bytes, 128 rows}, SWIZZLE_128B
 static bool make_w_map(CUtensorMap* out, const void* w, int n, int row_bytes) {
-  bind_primary_context();
-  EncodeTiledFn enc = get_encode();
-  if (!enc) { set_last_error(__FILE__, __LINE__, "cuTensorMapEncodeTiled unavailable"); return false; }
   cuuint64_t dims[2] = {(cuuint64_t)row_bytes, (cuuint64_t)n};
   cuuint64_t strides[1] = {(cuuint64_t)row_bytes};
   cuuint32_t box[2] = {128u, (cuuint32_t)BLOCK_N};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(w), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_last_error(__FILE__, __LINE__, ("weight-only gemm: cuTensorMapEncodeTiled failed: " + std::to_string((int)r)).c_str()); return false; }
-  return true;
-}
-
-static uint32_t make_idesc(bool bf16, int ntok) {
-  uint32_t d = 0;
-  d |= 1u << 4;                                  // fp32 accumulate
-  d |= (bf16 ? 1u : 0u) << 7;                    // A (dequantised weights, TMEM) in the activation dtype: mixed f16 x bf16 traps
-  d |= (bf16 ? 1u : 0u) << 10;                   // B (activations)
-  d |= (uint32_t)(ntok >> 3) << 17;              // UMMA N = tokens
-  d |= (uint32_t)(BLOCK_N >> 4) << 24;           // UMMA M = 128 channels
-  return d;
+  return encode_tiled(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, w, dims, strides, box, "weight-only gemm");
 }
 
 template <int NTOK, int G, int WST, int XPER, bool INT4, bool BF16>
@@ -421,7 +383,9 @@ static int launch(const WoGemmArgs& g, const CUtensorMap& mw, cudaStream_t s) {
   p.splits = splits;
   p.kb_per_split = kb_per;
   p.scale = g.scale; p.bias = g.bias; p.out = g.out; p.bf16 = g.bf16;
-  p.idesc = make_idesc(g.bf16, NTOK);
+  // UMMA M = 128 channels, N = tokens; A (dequantised weights, TMEM) in the activation dtype: mixed f16 x bf16 traps
+  const uint32_t f = g.bf16 ? 1u : 0u;
+  p.idesc = umma_idesc(f, f, false, false, BLOCK_N, NTOK, false);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(n_tiles, splits, t_tiles); cfg.blockDim = dim3(wo_threads(G)); cfg.dynamicSmemBytes = SMEM; cfg.stream = s;
   cudaLaunchAttribute at[1];

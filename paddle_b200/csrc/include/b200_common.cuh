@@ -65,6 +65,35 @@ template <typename T> __device__ __forceinline__ void st16_stream(T* p, const Ve
                : "memory");
 }
 
+// ---- GEMM epilogue
+__device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.f + erff(x * 0.70710678118654752f)); }
+
+// 32 consecutive outputs of one row (the first `valid` of them in bounds), stored or added to what is there: 16-byte vectors when the
+// chunk is whole and aligned, element by element otherwise
+template <typename TO>
+__device__ __forceinline__ void store_row_chunk(TO* __restrict__ dst, const float (&v)[32], int valid, bool accumulate) {
+  if (valid >= 32 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
+    constexpr int N = Vec16<TO>::N;
+#pragma unroll
+    for (int q = 0; q < 32 / N; ++q) {
+      Vec16<TO> o;
+      if (accumulate) {
+        Vec16<TO> old = ld16(dst + q * N);
+#pragma unroll
+        for (int j = 0; j < N; ++j) o.v[j] = from_f<TO>(v[q * N + j] + to_f(old.v[j]));
+      } else {
+#pragma unroll
+        for (int j = 0; j < N; ++j) o.v[j] = from_f<TO>(v[q * N + j]);
+      }
+      st16(dst + q * N, o);
+    }
+  } else {
+#pragma unroll
+    for (int j = 0; j < 32; ++j)
+      if (j < valid) dst[j] = from_f<TO>(accumulate ? v[j] + to_f(dst[j]) : v[j]);
+  }
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -1,8 +1,12 @@
 // Blackwell (sm_100a) PTX wrappers shared by every tcgen05 / TMA kernel: mbarriers (with a bounded wait that traps instead of hanging
-// the GPU), proxy / tcgen05 fences, TMA tile and bulk copies, UMMA issue + commit, shared-memory matrix descriptors, TMEM loads / stores.
-// One definition: a protocol fix is made once.  (CTA-pair and peer-memory variants that only gemm_sm100_2cta.cu uses stay there.)
+// the GPU), proxy / tcgen05 fences, cluster (CTA-pair) addressing, TMA tile and bulk copies, stores and reductions, UMMA issue + commit
+// for cta_group::1 and ::2, shared-memory matrix descriptors, TMEM allocation / loads / stores, and the release / acquire flags and
+// bounded spin of the cross-rank epoch protocols.
+// One definition: a protocol fix is made once.
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cstdint>
 #include <cstdio>
 
@@ -55,6 +59,27 @@ __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::
 __device__ __forceinline__ void cluster_sync() {
   asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+// the same shared-memory offset in cluster CTA `rank` (an address for ld / st.shared::cluster)
+__device__ __forceinline__ uint32_t mapa(uint32_t addr, uint32_t rank) {
+  uint32_t r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
+  return r;
+}
+// arrive on the barrier at the same smem offset in cluster CTA `rank`
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar, uint32_t rank) {
+  asm volatile(
+      "{\n\t.reg .b32 ra;\n\t"
+      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
+      "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}"
+      ::"r"(bar), "r"(rank)
+      : "memory");
+}
+constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;   // clears the CTA-rank bit of a shared::cluster address
 
 // ---------------------------------------------------------------------------------------------- TMA
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
@@ -81,9 +106,53 @@ __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* map
       ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
       : "memory");
 }
+// TMA load whose completion bytes are credited to the LEADER CTA's mbarrier (CTA pair)
+__device__ __forceinline__ void tma_load_3d_2sm(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, int c2, uint64_t hint) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
+      " [%0], [%1, {%3, %4, %5}], [%2], %6;"
+      ::"r"(dst), "l"(map), "r"(bar & kPeerBitMask), "r"(c0), "r"(c1), "r"(c2), "l"(hint)
+      : "memory");
+}
 // contiguous bytes global -> shared, completion on an mbarrier
 __device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
+}
+// smem box -> global (or peer) memory; completion tracked by the issuing thread's bulk async-group
+__device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, uint32_t src, int c0, int c1, int c2) {
+  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
+               ::"l"(map), "r"(src), "r"(c0), "r"(c1), "r"(c2)
+               : "memory");
+}
+// same box, but added to the destination (bf16 / fp16 / fp32 add performed by the L2 reduction units): D += tile without reading D
+__device__ __forceinline__ void tma_reduce_add_3d(const CUtensorMap* map, uint32_t src, int c0, int c1, int c2) {
+  asm volatile("cp.reduce.async.bulk.tensor.3d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3, %4}], [%1];"
+               ::"l"(map), "r"(src), "r"(c0), "r"(c1), "r"(c2)
+               : "memory");
+}
+// BYTES contiguous fp32 in shared memory added to global memory by the L2 reduction units (bulk async-group)
+template <uint32_t BYTES>
+__device__ __forceinline__ void bulk_reduce_add_f32(float* dst, uint32_t src) {
+  asm volatile("cp.reduce.async.bulk.global.shared::cta.bulk_group.add.f32 [%0], [%1], %2;" ::"l"(dst), "r"(src), "n"(BYTES) : "memory");
+}
+__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// at most N of this thread's bulk groups are still pending: complete (wait), or done reading their shared memory (wait_read)
+template <int N> __device__ __forceinline__ void bulk_wait() { asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory"); }
+template <int N> __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
+
+// ---------------------------------------------------------------------------------------------- shared-memory stores
+__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
+  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
+}
+// two floats -> one 32-bit register of T (bf16 / fp16), one cvt.rn.{bf16x2,f16x2}.f32
+template <typename T> __device__ __forceinline__ uint32_t pack2(float a, float b);
+template <> __device__ __forceinline__ uint32_t pack2<__nv_bfloat16>(float a, float b) {
+  __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
+  return *reinterpret_cast<uint32_t*>(&v);
+}
+template <> __device__ __forceinline__ uint32_t pack2<__half>(float a, float b) {
+  __half2 v = __floats2half2_rn(a, b);
+  return *reinterpret_cast<uint32_t*>(&v);
 }
 
 // ---------------------------------------------------------------------------------------------- UMMA (cta_group::1)
@@ -143,7 +212,41 @@ __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
 
+// ---------------------------------------------------------------------------------------------- UMMA (cta_group::2, CTA pair)
+// issued by the leader CTA; A and B are read from both CTAs' shared memory, D spans both CTAs' TMEM
+__device__ __forceinline__ void umma_f16_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// commit -> arrive on the barrier at this offset in BOTH CTAs of the pair
+__device__ __forceinline__ void umma_commit_2sm(uint32_t bar) {
+  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+               ::"r"(bar), "h"((uint16_t)0x3)
+               : "memory");
+}
+
 // ---------------------------------------------------------------------------------------------- TMEM
+// Allocation by one whole warp: the base address of `cols` columns (a power of two >= 32) is written to shared memory at `dst`.
+// CG = 2: one allocation across the CTA pair (both CTAs' warps execute it).  The permit is given up right away: one allocation per CTA.
+template <int CG = 1>
+__device__ __forceinline__ void tmem_alloc(uint32_t dst, uint32_t cols) {
+  if constexpr (CG == 1) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst), "r"(cols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  } else {
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst), "r"(cols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+  }
+}
+template <int CG = 1>
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
+  if constexpr (CG == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
+  else asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
+}
 // 32 rows x 128 bits of shared memory -> 4 TMEM columns, replicated into the four 32-lane quadrants
 __device__ __forceinline__ void tmem_cp_sf(uint32_t tmem_dst, uint64_t sdesc) {
   asm volatile("tcgen05.cp.cta_group::1.32x128b.warpx4 [%0], %1;" ::"r"(tmem_dst), "l"(sdesc) : "memory");
@@ -187,6 +290,35 @@ __device__ __forceinline__ float ex2(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
+}
+
+// ---------------------------------------------------------------------------------------------- cross-rank / cross-CTA flags
+__device__ __forceinline__ void st_release_sys_u32(uint32_t* p, uint32_t v) {
+  asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __forceinline__ uint32_t ld_acquire_sys_u32(const uint32_t* p) {
+  uint32_t v;
+  asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ uint32_t ld_acquire_gpu_u32(const uint32_t* p) {
+  uint32_t v;
+  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+// Bounded spin until the epoch flag at `p` (published with st_release_sys_u32, possibly by a peer GPU) reaches `target`.  Epochs only
+// grow; the signed distance survives wrap-around.  A dead peer or a protocol bug must not hang the GPU: after kSpinTimeoutNs the thread
+// prints the caller's message `fmt` (which names its protocol) with `args` and traps.
+constexpr uint64_t kSpinTimeoutNs = 10000000000ull;   // 10 s
+template <typename... Args>
+__device__ __forceinline__ void spin_sys_ge(const uint32_t* p, uint32_t target, const char* fmt, Args... args) {
+  const uint64_t t0 = globaltimer_ns();
+  while ((int32_t)(ld_acquire_sys_u32(p) - target) < 0) {
+    if (globaltimer_ns() - t0 > kSpinTimeoutNs) {
+      printf(fmt, args...);
+      __trap();
+    }
+  }
 }
 
 }  // namespace ptx

@@ -25,7 +25,8 @@ def rel_err(a, b):
 
 
 @pytest.mark.parametrize("a_km,b_nk", [(False, False), (False, True), (True, False), (True, True)])
-@pytest.mark.parametrize("m,n,k", [(256, 512, 256), (384, 320, 192), (128, 64, 64), (1000, 776, 520), (4096, 5120, 1024)])
+# (512, 300, 256): with b_nk the CTA-pair kernel writes 600-byte output rows, which only its register-store epilogue can handle
+@pytest.mark.parametrize("m,n,k", [(256, 512, 256), (384, 320, 192), (128, 64, 64), (1000, 776, 520), (4096, 5120, 1024), (512, 300, 256)])
 @pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float16])
 def test_gemm_layouts(a_km, b_nk, m, n, k, dtype):
     torch.manual_seed(0)
